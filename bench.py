@@ -4,6 +4,7 @@ decode of 30 s chunks (BASELINE.json metric), one process per GPU.
 
     python bench.py --gpus N --steps K --warmup W             # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W      # the reference algorithm on the host cores
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # + the last timed step's hypotheses, DIR/*.npy
 
 A "step" = one recording of N x `--chunks` (default 64) 30 s chunks, chunk-sharded over the N ranks (contiguous
 blocks, reverb_b200/dist.py): every rank runs
@@ -281,6 +282,35 @@ def parity_vs_cpu(asr, eng, model, cpu) -> dict:
     }
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, hyps, max_tok: int) -> None:
+    """Writes the hypotheses of one step to out_dir/<name>.npy as float64, one row per chunk in chunk order
+    (`chunk`), token-indexed arrays padded with -1 after `num_tokens` entries.  Above DUMP_LIMIT_BYTES a fixed,
+    seeded sample of the chunks is written instead, so two builds given the same arguments dump the same rows."""
+    rows = np.arange(len(hyps))
+    row_bytes = 8 * (4 + 3 * max_tok)
+    if len(rows) * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    out = {"chunk": rows.astype(np.float64), "num_tokens": np.empty(len(rows)), "score": np.empty(len(rows)),
+           "confidence": np.empty(len(rows))}
+    for name in ("tokens", "times", "tokens_confidence"):
+        out[name] = np.full((len(rows), max_tok), -1.0)
+    for i, c in enumerate(rows):
+        h = hyps[c]
+        n = len(h.tokens)
+        out["num_tokens"][i], out["score"][i], out["confidence"][i] = n, float(h.score), float(h.confidence)
+        out["tokens"][i, :n] = h.tokens
+        if h.times is not None:
+            out["times"][i, :len(h.times)] = h.times
+        if h.tokens_confidence is not None:
+            out["tokens_confidence"][i, :n] = h.tokens_confidence
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _claim_stdout():
     """Only the JSON line may reach stdout: libraries (NCCL prints its version there) are redirected to stderr."""
     sys.stdout.flush()
@@ -314,7 +344,13 @@ def main():
                     help="after warm-up run ONE step between cudaProfilerStart/Stop and exit (for `ncu --profile-from-start off`)")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling (configs[2]) record")
     ap.add_argument("--breakdown", action="store_true", help="print a per-stage wall-clock split (synchronised) to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the hypotheses of the last timed step (every rank's chunks) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "rvb":
+        ap.error("--dump-outputs applies to the CUDA path (--impl rvb)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -489,6 +525,8 @@ def main():
     assert len(recs) == args.steps and len(got) == args.chunks * world, (len(recs), len(got))
     mine = got[rank * args.chunks:(rank + 1) * args.chunks]
     assert all(list(a.tokens) == list(b.tokens) and a.times == b.times for a, b in zip(mine, hyps)), "all-gather corrupted the records"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, got, max_tok)
 
     # end-to-end through the host API (pinned host PCM in, host hypotheses out)
     run_steps(1, True)

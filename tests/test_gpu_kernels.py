@@ -33,7 +33,7 @@ def _check(lib, rc):
 def test_fbank_matches_oracle_and_torchaudio_golden(lib):
     from oracle import fbank_np
     from reverb_b200 import synth
-    gold = dict(np.load("tests/golden/fbank.npz"))
+    gold = dict(np.load(os.path.join(os.path.dirname(__file__), "golden", "fbank.npz")))
     for key, ref in gold.items():
         n = int(key.split("_")[0][1:])
         seed = int(key.split("seed")[1])

@@ -1,15 +1,19 @@
 """The CPU oracle (oracle/) vs the committed outputs of the live reference (tests/golden): the oracle
 must reproduce the reference bit for bit on the model graph / searches (same ATen CPU ops, same float
 semantics) and to fp32 round-off on fbank (numpy vs torchaudio FFT)."""
+import os
+
 import numpy as np
 import pytest
 import torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_fbank_oracle_vs_torchaudio_golden():
     from oracle import fbank_np
     from reverb_b200 import synth
-    gold = dict(np.load("tests/golden/fbank.npz"))
+    gold = dict(np.load(os.path.join(GOLDEN, "fbank.npz")))
     assert len(gold) >= 5
     for key, ref in gold.items():
         n = int(key.split("_")[0][1:])
@@ -60,7 +64,7 @@ def test_oracle_attention_mode_vs_reference_golden(golden_cases, model_dirs, cas
     token ids the live reference returned (tests/golden/attention_mode.json, oracle/make_golden_attention.py)."""
     import json
     from oracle import pipeline_ref
-    gold = json.load(open("tests/golden/attention_mode.json"))["cases"][case]
+    gold = json.load(open(os.path.join(GOLDEN, "attention_mode.json")))["cases"][case]
     meta, arr = golden_cases[case]
     d, _ = model_dirs[case]
     orc = pipeline_ref.OracleASR(d)
@@ -78,8 +82,8 @@ def test_oracle_bounded_context_encoder_vs_reference_golden(golden_cases, model_
     reproduce the live reference (tests/golden/chunked.*, oracle/make_golden_chunked.py) bit for bit."""
     import json
     from oracle import pipeline_ref
-    gold = json.load(open("tests/golden/chunked.json"))
-    arr_c = dict(np.load("tests/golden/chunked.npz"))
+    gold = json.load(open(os.path.join(GOLDEN, "chunked.json")))
+    arr_c = dict(np.load(os.path.join(GOLDEN, "chunked.npz")))
     meta, arr = golden_cases[case]
     orc = pipeline_ref.OracleASR(model_dirs[case][0])
     cat = torch.tensor([meta["verbatimicity"], 1.0 - meta["verbatimicity"]])
@@ -95,7 +99,7 @@ def test_oracle_bounded_context_encoder_vs_reference_golden(golden_cases, model_
 
 
 def _resample_cases():
-    gold = dict(np.load("tests/golden/resample.npz"))
+    gold = dict(np.load(os.path.join(GOLDEN, "resample.npz")))
     for key, ref in gold.items():
         rate = int(key.split("_")[0][1:])
         n = int(key.split("_")[1][1:])
@@ -148,8 +152,8 @@ def test_oracle_streaming_cache_pass_vs_reference_golden(golden_cases, model_dir
     pass (chunk mask, all frames valid) is the same function — the identity the engine's simulate_streaming relies on."""
     import json
     from oracle import model_ref, pipeline_ref
-    gold = json.load(open("tests/golden/streaming.json"))
-    arr_s = dict(np.load("tests/golden/streaming.npz"))
+    gold = json.load(open(os.path.join(GOLDEN, "streaming.json")))
+    arr_s = dict(np.load(os.path.join(GOLDEN, "streaming.npz")))
     meta, arr = golden_cases[case]
     orc = pipeline_ref.OracleASR(model_dirs[case][0])
     feats = torch.from_numpy(arr["feats"][:gold["frames"]]).unsqueeze(0)
